@@ -1,7 +1,10 @@
 """bench.py -- headline metric of BASELINE.json on B200: whisper-large-v3 tokens/sec (and RTF) on 30 s chunks.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR writes what the last timed step computed (rank 0's chunks) as DIR/<name>.npy; the inputs are seeded, so two
+builds run with the same arguments can be compared output for output.
 
 A "step" is one pass of the hot path over one batch of synthetic 30 s chunks on every rank:
 PCM -> log-mel -> 32-layer encoder -> cross K/V -> `new_tokens` greedy decoder steps -> token ids.
@@ -181,7 +184,10 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="b200 arm: write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -277,6 +283,8 @@ def main():
     if rank == 0:
         sampler.start()
     ms_res = timed(step_resident, args.steps, args.warmup)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng, A, prompt.shape[1])
     k0 = eng.decode_kernel_launches()
     ms_e2e = timed(step_e2e, args.steps, args.warmup)
     # decoder kernels of ONE e2e step, counted from the captured step graphs (warm-up steps included in the delta)
@@ -375,6 +383,19 @@ def main():
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir: str, eng, A: int, plen: int) -> None:
+    """What the last resident step left in the engine, read back the way a caller of that path reads it: the generated token
+    ids (float64, exact), the logits of the last decoder step and the encoder output (float32).  About 8 MB at large-v3 dims."""
+    toks, _, _ = eng.decode_read()
+    arrays = {"tokens": toks[:A, plen:plen + NEW_TOKENS].astype(np.float64),
+              "logits": eng.logits()[:A].cpu().numpy(),
+              "encoder_out": eng.encoder_output(A).cpu().numpy()}
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def extra_configs(model, weights, dev, rank, world, dist):

@@ -11,7 +11,7 @@
 #   configs      tools/bench_configs.py C3 C5 C4 (BASELINE.json configs bench.py does not time)
 #   ncu_batched  launch list + ncu --set full of the batched decoder step (A = 64)
 #   steptime     CUDA-event time of one decoder step at several (audios, beams, chunk length) shapes
-cd "${GRAFT_REPO_ROOT:-/root/repo}"
+cd "$(dirname "$0")/.."
 mkdir -p gpurun_out
 export PYTHONPATH=$PWD TRANSFORMERS_OFFLINE=1 HF_HUB_OFFLINE=1 TOKENIZERS_PARALLELISM=false
 TAG=${1:-r2}; shift

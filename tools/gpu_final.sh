@@ -1,6 +1,6 @@
 #!/bin/bash
 # Last check of a round: the suites that exercise bw_encode's graph replay (several batch sizes, seek-loop re-encodes) + smoke().
-cd "${GRAFT_REPO_ROOT:-/root/repo}"
+cd "$(dirname "$0")/.."
 mkdir -p gpurun_out
 export PYTHONPATH=$PWD TRANSFORMERS_OFFLINE=1 HF_HUB_OFFLINE=1 TOKENIZERS_PARALLELISM=false
 O=gpurun_out/${1:-final}

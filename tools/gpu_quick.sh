@@ -2,7 +2,7 @@
 # A short, hang-proof check (every step under its own tight timeout): default paths first, then the encoder switches.
 # (r2o ran this with the 16-warp GEMM epilogue as well; that variant measured slower and is gone.)
 #     gpurun --timeout 480 -- 'bash tools/gpu_quick.sh <tag>'
-cd "${GRAFT_REPO_ROOT:-/root/repo}"
+cd "$(dirname "$0")/.."
 mkdir -p gpurun_out
 export PYTHONPATH=$PWD TRANSFORMERS_OFFLINE=1 HF_HUB_OFFLINE=1 TOKENIZERS_PARALLELISM=false
 O=gpurun_out/${1:-quick}
