@@ -186,6 +186,19 @@ int bw_op_layernorm(const float* x, const float* g, const float* b, void* out, i
 /* out[M,N] fp32 = epi(LN?(x[M,K]) W[N,K]^T), M <= 8 */
 int bw_op_gemv(const float* x, const float* ln_g, const float* ln_b, const void* W, int32_t M, int32_t N, int32_t K,
                const float* bias, float alpha, int32_t act, const float* residual, float* out, void* stream);
+/* causal self-attention of one decoder step over positions 0..*pos. qkv [Q,3D] fp32 (q pre-scaled), or nsplit raw partial sums
+   [nsplit][Q][3D] + qkv_bias, q scaled by q_alpha (batched path). append = 1: the k/v of this step are rounded to 16 bit and written
+   to kc/vc at *pos (batched path). anc [Q,Tmax] or NULL. elem_dtype 0 = bf16, 1 = fp16 (dispatch to the _bf16 / _f16 build). */
+int bw_op_self_attn(const float* qkv, int32_t nsplit, const float* qkv_bias, float q_alpha, void* kc, void* vc, const int32_t* anc,
+                    int32_t append, void* out, int32_t out_is_f32, const int32_t* pos_dev, int32_t Q, int32_t H, int32_t Tmax,
+                    int32_t elem_dtype, void* stream);
+/* cross-attention of A*G query rows over kc/vc [A,H,S,64]. impl 0 = the engine's policy, 1 = split kernel, 2 = streaming kernel.
+   part_o / part_ml / counters: caller-owned scratch of the sizes in decode.cuh; counters must be zero on entry and are zero on
+   return. align / head_slots / Ha / Tcap / step_base: the word-timestamp capture (align may be NULL). */
+int bw_op_cross_attn(const float* q, int32_t nsplit, const float* q_bias, float q_alpha, const void* kc, const void* vc,
+                     void* out, int32_t out_is_f32, float* part_o, float* part_ml, uint32_t* counters, int32_t A, int32_t G,
+                     int32_t H, int32_t S, float* align, const int32_t* head_slots, int32_t Ha, int32_t Tcap, int32_t step_base,
+                     const int32_t* pos_dev, int32_t impl, int32_t elem_dtype, void* stream);
 
 #ifdef __cplusplus
 }

@@ -33,6 +33,8 @@ pytestmark = pytest.mark.gpu
 LOGIT_CAP_SIGMA = 0.30
 ENC_TOL = {"turbo10": (0.30, 0.045), "large30": (0.30, 0.035)}  # (max abs, mean abs) of the final-LayerNorm output (unit scale)
 SEEDS = (1000, 1001, 1002, 1003)
+# step-path switches an engine reads once, when it is created: part of the engine cache key, so a test that sets one gets a fresh engine
+PATH_SWITCHES = ("BW_NO_MEGA", "BW_BATCH_MIN", "BW_XATTN_STREAM_MIN")
 
 
 class Case:
@@ -57,7 +59,7 @@ class Case:
     def engine(self, max_audios, dtype=torch.bfloat16):
         from thewhisper_b200.engine import ModelDims, WhisperEngine
 
-        key = (max_audios, dtype)
+        key = (max_audios, dtype, tuple(os.environ.get(k) for k in PATH_SWITCHES))
         for k in list(self._engines):  # one engine alive at a time (cross K/V of 64 audios = 15.7 GB)
             if k != key:
                 self._engines.pop(k).close()
@@ -142,8 +144,10 @@ def test_encoder_at_benchmark_dims(cuda, case):
     assert e1.max() < mx and e1.mean() < mean, (e1.max(), e1.mean())
 
 
-def _decode_check(case, Q, monkeypatch, env=None, dtype=torch.bfloat16):
-    """Teacher-forced logits at every position + free-running greedy (tie-aware) for Q sequences over audios SEEDS[q % 4]."""
+def _decode_check(case, Q, monkeypatch, env=None, dtype=torch.bfloat16, want_path=None):
+    """Teacher-forced logits at every position + free-running greedy (tie-aware) for Q sequences over audios SEEDS[q % 4].
+    want_path: the decoder step path ('mega' / 'perop' / 'batched') the teacher-forced steps must have run."""
+    from tests.test_decoder_attn_gpu import step_path
     from thewhisper_b200 import synthetic as S
 
     for k, v in (env or {}).items():
@@ -163,6 +167,7 @@ def _decode_check(case, Q, monkeypatch, env=None, dtype=torch.bfloat16):
     uniq = sorted(set(seeds))
     refs = {s: case.oracle_tf(s, ids.tolist()) for s in uniq if s != 1000}
     first_row = {s: seeds.index(s) for s in uniq}
+    launches0 = eng.decode_kernel_launches()
     for t in range(len(ids)):
         eng.decode_run(1)
         lg = eng.logits().cpu().numpy()
@@ -179,6 +184,8 @@ def _decode_check(case, Q, monkeypatch, env=None, dtype=torch.bfloat16):
                 worst = max(worst, float(np.abs(lg[q] - ref_row).max()))
                 top = np.argsort(-ref_row)[:8]
                 worst_top = max(worst_top, float(np.abs(lg[q][top] - ref_row[top]).max()))
+    if want_path is not None:
+        assert step_path(eng, launches0, len(ids)) == want_path
     worst = max(worst, worst_top)
     hf_err = case.hf_bf16_err(1001, ids.tolist())
     print(f"\n[{case.tag} Q={Q} {env or 'default'} {str(dtype).replace('torch.', '')}] teacher-forced max |dlogit| = {worst:.4f} = {worst / sigma:.4f} sigma (sigma {sigma:.3f}); "
@@ -240,7 +247,7 @@ def test_decoder_batched_at_benchmark_dims(cuda, case, Q, monkeypatch):
 @pytest.mark.parametrize("case", ["large30"], indirect=True)
 def test_decoder_perop_q1_at_benchmark_dims(cuda, case, monkeypatch):
     """The per-op kernels at Q = 1 (BW_NO_MEGA=1): what beams and the timestamp rules run."""
-    _decode_check(case, 1, monkeypatch, env={"BW_NO_MEGA": "1"})
+    _decode_check(case, 1, monkeypatch, env={"BW_NO_MEGA": "1"}, want_path="perop")
 
 
 @pytest.mark.parametrize("case", ["large30"], indirect=True)

@@ -74,6 +74,8 @@ SYMBOLS = {
     "bw_op_attn_enc": (C.c_int, [_P, _P, _P, _I, _I, _I, _I, _P]),
     "bw_op_layernorm": (C.c_int, [_P, _P, _P, _P, _I, _I, _I, _P]),
     "bw_op_gemv": (C.c_int, [_P, _P, _P, _P, _I, _I, _I, _P, _F, _I, _P, _P, _P]),
+    "bw_op_self_attn": (C.c_int, [_P, _I, _P, _F, _P, _P, _P, _I, _P, _I, _P, _I, _I, _I, _I, _P]),
+    "bw_op_cross_attn": (C.c_int, [_P, _I, _P, _F, _P, _P, _P, _I, _P, _P, _P, _I, _I, _I, _I, _P, _P, _I, _I, _I, _P, _I, _I, _P]),
 }
 
 _lib: Optional[C.CDLL] = None

@@ -148,4 +148,27 @@ int bw_op_gemv(const float* x, const float* ln_g, const float* ln_b, const void*
   return bw_op_gemv_bf16(x, ln_g, ln_b, W, M, N, K, bias, alpha, act, residual, out, stream);
 }
 
+// ---- single ops with a 16-bit cache operand: the build elem_dtype names ---------------------------------------------------------
+int bw_op_self_attn(const float* qkv, int32_t nsplit, const float* qkv_bias, float q_alpha, void* kc, void* vc, const int32_t* anc,
+                    int32_t append, void* out, int32_t out_is_f32, const int32_t* pos_dev, int32_t Q, int32_t H, int32_t Tmax,
+                    int32_t elem_dtype, void* stream) {
+  g_last_f16 = elem_dtype == 1;
+  if (elem_dtype == 1)
+    return bw_op_self_attn_f16(qkv, nsplit, qkv_bias, q_alpha, kc, vc, anc, append, out, out_is_f32, pos_dev, Q, H, Tmax, elem_dtype, stream);
+  // an unknown elem_dtype: the bf16 build reports it
+  return bw_op_self_attn_bf16(qkv, nsplit, qkv_bias, q_alpha, kc, vc, anc, append, out, out_is_f32, pos_dev, Q, H, Tmax,
+                              elem_dtype, stream);
+}
+int bw_op_cross_attn(const float* q, int32_t nsplit, const float* q_bias, float q_alpha, const void* kc, const void* vc,
+                     void* out, int32_t out_is_f32, float* part_o, float* part_ml, uint32_t* counters, int32_t A, int32_t G,
+                     int32_t H, int32_t S, float* align, const int32_t* head_slots, int32_t Ha, int32_t Tcap, int32_t step_base,
+                     const int32_t* pos_dev, int32_t impl, int32_t elem_dtype, void* stream) {
+  g_last_f16 = elem_dtype == 1;
+  if (elem_dtype == 1)
+    return bw_op_cross_attn_f16(q, nsplit, q_bias, q_alpha, kc, vc, out, out_is_f32, part_o, part_ml, counters, A, G, H, S, align,
+                                head_slots, Ha, Tcap, step_base, pos_dev, impl, elem_dtype, stream);
+  return bw_op_cross_attn_bf16(q, nsplit, q_bias, q_alpha, kc, vc, out, out_is_f32, part_o, part_ml, counters, A, G, H, S, align,
+                               head_slots, Ha, Tcap, step_base, pos_dev, impl, elem_dtype, stream);
+}
+
 }  // extern "C"

@@ -1062,4 +1062,41 @@ int bw_op_gemv(const float* x, const float* ln_g, const float* ln_b, const void*
   return launch_gemv(static_cast<cudaStream_t>(stream), g);
 }
 
+int bw_op_self_attn(const float* qkv, int32_t nsplit, const float* qkv_bias, float q_alpha, void* kc, void* vc, const int32_t* anc,
+                    int32_t append, void* out, int32_t out_is_f32, const int32_t* pos_dev, int32_t Q, int32_t H, int32_t Tmax,
+                    int32_t elem_dtype, void* stream) {
+  BW_CHECK(qkv && kc && vc && out && pos_dev, "bw_op_self_attn: null pointer");
+  BW_CHECK(Q >= 1 && H >= 1 && Tmax >= 1 && nsplit >= 0, "bw_op_self_attn: Q=%d H=%d Tmax=%d nsplit=%d out of range", Q, H, Tmax, nsplit);
+  BW_CHECK(elem_dtype == 0 || elem_dtype == 1, "bw_op_self_attn: elem_dtype=%d must be 0 (bf16) or 1 (fp16)", elem_dtype);
+  const int D = H * 64;
+  SelfAttnArgs s;
+  s.qkv = qkv; s.nsplit = nsplit; s.split_stride = (long long)Q * 3 * D; s.qkv_bias = qkv_bias; s.q_alpha = q_alpha;
+  s.kc = static_cast<const bf16*>(kc); s.vc = static_cast<const bf16*>(vc); s.anc = anc; s.pos = pos_dev;
+  if (append) { s.kc_w = static_cast<bf16*>(kc); s.vc_w = static_cast<bf16*>(vc); }
+  if (out_is_f32) s.out = static_cast<float*>(out);
+  else s.out_bf16 = static_cast<bf16*>(out);
+  s.H = H; s.D = D; s.Tmax = Tmax;
+  return launch_self_attn(static_cast<cudaStream_t>(stream), s, Q);
+}
+
+int bw_op_cross_attn(const float* q, int32_t nsplit, const float* q_bias, float q_alpha, const void* kc, const void* vc,
+                     void* out, int32_t out_is_f32, float* part_o, float* part_ml, uint32_t* counters, int32_t A, int32_t G,
+                     int32_t H, int32_t S, float* align, const int32_t* head_slots, int32_t Ha, int32_t Tcap, int32_t step_base,
+                     const int32_t* pos_dev, int32_t impl, int32_t elem_dtype, void* stream) {
+  BW_CHECK(q && kc && vc && out, "bw_op_cross_attn: null pointer");
+  BW_CHECK(impl == 2 || (part_o && part_ml && counters), "bw_op_cross_attn: the split kernel needs part_o, part_ml and counters");
+  BW_CHECK(!align || (head_slots && pos_dev && Ha >= 1 && Tcap >= 1), "bw_op_cross_attn: align needs head_slots, pos_dev, Ha and Tcap");
+  BW_CHECK(A >= 1 && H >= 1 && S >= 1 && nsplit >= 0, "bw_op_cross_attn: A=%d H=%d S=%d nsplit=%d out of range", A, H, S, nsplit);
+  BW_CHECK(elem_dtype == 0 || elem_dtype == 1, "bw_op_cross_attn: elem_dtype=%d must be 0 (bf16) or 1 (fp16)", elem_dtype);
+  CrossAttnArgs c;
+  c.q = q; c.nsplit = nsplit; c.split_stride = (long long)A * G * H * 64; c.q_bias = q_bias; c.q_alpha = q_alpha;
+  c.kc = static_cast<const bf16*>(kc); c.vc = static_cast<const bf16*>(vc);
+  if (out_is_f32) c.out = static_cast<float*>(out);
+  else c.out_bf16 = static_cast<bf16*>(out);
+  c.part_o = part_o; c.part_ml = part_ml; c.counters = counters;
+  c.S = S; c.H = H; c.D = H * 64; c.G = G; c.pos = pos_dev;
+  c.align = align; c.head_slots = head_slots; c.Ha = Ha; c.Tcap = Tcap; c.step_base = step_base;
+  return launch_cross_attn(static_cast<cudaStream_t>(stream), c, A, impl);
+}
+
 }  // extern "C"

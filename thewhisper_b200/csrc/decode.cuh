@@ -148,7 +148,8 @@ extern int g_mega_coop;  // 1: the persistent step kernels are launched cooperat
 int launch_gemv(cudaStream_t st, const GemvArgs& a);
 int launch_embed(cudaStream_t st, const bf16* E, const float* P, const int* tokens, const int* pos, float* x, int Q, int D, int Tmax);
 int launch_self_attn(cudaStream_t st, const SelfAttnArgs& a, int Q);
-int launch_cross_attn(cudaStream_t st, const CrossAttnArgs& a, int A);
+// impl: 0 = the engine's policy (streaming kernel from BW_XATTN_STREAM_MIN CTAs, default 296), 1 = split kernel, 2 = streaming kernel
+int launch_cross_attn(cudaStream_t st, const CrossAttnArgs& a, int A, int impl = 0);
 int launch_select(cudaStream_t st, const SelectArgs& a);
 // x[q] += bias + sum_{s < nsplit} part[s][q]  (fixed order: deterministic), then y[q] = LayerNorm(x[q]) as bf16.
 // nsplit = 0: LayerNorm only.  part: [nsplit][Q][D] fp32 partial sums of a split-K GEMM (gemm_tc_split).

@@ -754,9 +754,10 @@ int launch_self_attn(cudaStream_t st, const SelfAttnArgs& a, int Q) {
   return 0;
 }
 
-int launch_cross_attn(cudaStream_t st, const CrossAttnArgs& a, int A) {
+int launch_cross_attn(cudaStream_t st, const CrossAttnArgs& a, int A, int impl) {
   BW_CHECK(a.G >= 1 && a.G <= MAXG, "cross_attn: G=%d must be in 1..%d", a.G, MAXG);
   BW_CHECK(a.S <= XSPLIT * XK, "cross_attn: S=%d exceeds %d", a.S, XSPLIT * XK);
+  BW_CHECK(impl >= 0 && impl <= 2, "cross_attn: impl=%d must be 0 (policy), 1 (split) or 2 (streaming)", impl);
   constexpr size_t smem1 = 2 * XK * 128 + (size_t)(1 * XK + 16 * 1 * 64) * sizeof(float);
   constexpr size_t smemG = 2 * XK * 128 + (size_t)(MAXG * XK + 16 * MAXG * 64) * sizeof(float);
   static bool attr = false;
@@ -768,7 +769,8 @@ int launch_cross_attn(cudaStream_t st, const CrossAttnArgs& a, int A) {
     // CTAs (A * H) from which the streaming kernel is used; 0 = never.  (Read per launch: launches happen at graph capture only.)
     const char* ev = getenv("BW_XATTN_STREAM_MIN");
     const int stream_min = ev ? atoi(ev) : 296;
-    if (stream_min > 0 && A * a.H >= stream_min) {
+    const bool stream = impl == 2 || (impl == 0 && stream_min > 0 && A * a.H >= stream_min);
+    if (stream) {
       auto smem_of = [](int gm) { return (size_t)4 * XT * 128 + (size_t)(gm * XT + gm * 64 + gm * 4 + 8 * gm * 64) * sizeof(float); };
       // instantiated for the exact beam count (a bound of 8 with g < G predicates issued 8 / 5 of the instructions at beam 5)
 #define BW_XSTREAM(GMV)                                                                                                   \
